@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          # this framework
     python bench.py --impl reference --steps K --warmup W  # reference CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                 # + outputs of the last timed step as DIR/*.npy
 
 Workload (BASELINE.json metric / configs[2]): WDX10_rna004_v1_0 (2601 support
 vectors, 11 classes, L=25, window 15) on synthetic barcode fingerprints S1
@@ -35,6 +36,8 @@ MODEL = "WDX10_rna004_v1_0"
 METRIC = "reads/s demuxed (WDX10 DTW+SVC)"
 READS_PER_GPU = 12_500_000  # 100 M / 8
 SIGMA = 0.35
+DUMP_ROWS = 1 << 18         # --dump-outputs sample: 2^18 reads x (index, label, confidence, 11 probabilities, flags) x 8 B = 31 MB
+DUMP_SEED = 2024
 
 
 def load_params():
@@ -52,6 +55,20 @@ def synth_host(params, n, seed):
         idx = rng.integers(0, params.n_sv, size=r1 - r0)
         X[r0:r1] = params.sv[idx] + SIGMA * rng.standard_normal((r1 - r0, params.L))
     return X
+
+
+def dump_outputs(out_dir, n, arrays):
+    """Per-read results of the last timed step (what DeviceModel.predict returns: label, confidence, class probabilities,
+    guard flags) for a fixed, seeded sample of this rank's n reads, as float64 DIR/<name>.npy, plus the sampled read
+    indices.  The inputs are seeded as well, so two builds run with the same arguments can be compared file by file."""
+    import torch
+
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_ROWS, replace=False)) if n > DUMP_ROWS else np.arange(n)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "read_index.npy"), idx.astype(np.float64))
+    sel = torch.from_numpy(idx).cuda()
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.index_select(0, sel).cpu().numpy().astype(np.float64))
 
 
 class ClockSampler:
@@ -968,6 +985,8 @@ def run_ours(args):
     kms_all, kl_all = dm.last_kernel_ms()
     ms_per_step = ms_total / args.steps
     value = n_total / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:       # before anything below reuses the result buffers
+        dump_outputs(args.dump_outputs, n, {"labels": lab_d, "confidence": conf_d, "probabilities": prob_d, "flags": flags_d})
 
     # labels gathered host-side in shard order (the only cross-rank exchange of the path)
     labels_host = lab_d.cpu().numpy()
@@ -1291,7 +1310,13 @@ def main():
     ap.add_argument("--port-only", action="store_true", help="reference arm: time the C port even if baseline/_ref is present")
     ap.add_argument("--no-extras", dest="extras", action="store_false",
                     help="skip the secondary measurements (streaming latency, fingerprint stage)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (a seeded sample of rank 0's reads) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours (the reference arm sizes its sample from a timing probe)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: W >= 3
     if args.impl == "reference":

@@ -16,7 +16,7 @@ from conftest import GOLD
 from wdx_testutil import real4000_rows
 
 pytestmark = pytest.mark.gpu
-LOCAL = os.path.join(GOLD, "_local", "real4000_adc_rows.npz")
+MINIBATCH = 1000        # production minibatch size (the reference's parser default)
 
 
 @pytest.fixture(scope="module")
@@ -149,26 +149,24 @@ def _spc(g):
 
 
 def test_gpu_whole_test_file_raw_signal_to_barcode_calls(g4000, models):
-    """BASELINE.json configs[0], all 4000 reads of test_data/demux/4000_rna004.pod5 in the production minibatches of
-    1000 (file order), raw ADC rows -> `MinibatchDemuxer.run` (CNN -> validation -> hail mary / LLR -> fingerprint ->
-    DTW + SVC) with llr_fallback=None: detection verdict, boundaries, fingerprints (bit-identical) and barcode calls of
-    EVERY read equal the reference chain's.  One caveat, recorded in the fixture: where two EQUAL t-test scores compete
-    (106 reads have such ties, for 1 of them the outcome depends on the order) scipy's result hangs on numpy's unstable
-    argsort; the kernels use the stable order, and for that read the expected values are the oracle's stable-order ones.  Needs the int16 rows of all reads (tests/golden/_local, written by
-    oracle/make_golden_real4000.py; git-ignored because of its size, shipped with the working tree)."""
-    if not os.path.exists(LOCAL):
-        pytest.skip("tests/golden/_local/real4000_adc_rows.npz not present: run oracle/make_golden_real4000.py where /root/reference exists")
+    """BASELINE.json configs[0] on the reads of test_data/demux/4000_rna004.pod5 whose int16 rows the fixture keeps
+    (every read that leaves the plain CNN path, every 16th read and the tie read below: 439 of the 4000), in minibatches
+    of MINIBATCH, raw ADC rows -> `MinibatchDemuxer.run` (CNN -> validation -> hail mary / LLR -> fingerprint -> DTW + SVC)
+    with llr_fallback=None: detection verdict, boundaries, fingerprints (bit-identical) and barcode calls of every one of
+    them equal the reference chain's over the whole file.  One caveat, recorded in the fixture: where two EQUAL t-test
+    scores compete (106 reads have such ties, for 1 of them the outcome depends on the order) scipy's result hangs on
+    numpy's unstable argsort; the kernels use the stable order, and for that read the expected values are the oracle's
+    stable-order ones."""
     from warpdemux_b200.detect import cnn, combined
     from warpdemux_b200.file_proc import AdcBatch, MinibatchDemuxer
     from warpdemux_b200.models.dtw_svm import DTW_SVM
     from warpdemux_b200.sig_proc import FingerprintConfig
 
     g = g4000
-    with np.load(LOCAL) as z:
-        full = {k: z[k] for k in z.files}
-    idx, rows, adc, num = real4000_rows(g, full)
+    idx, rows, adc, num = real4000_rows(g)
     n = idx.size
-    assert n == 4000
+    off_path = (g["n_validate"] > 1) | (g["success"] == 0)
+    assert set(np.flatnonzero(off_path).tolist()) | set(g["stable_idx"].tolist()) <= set(idx.tolist())
     spc = _spc(g)
     md = cnn.load_cnn_model(os.path.join(GOLD, "models", "cnn_rna004_130bps_v0.2.4.npz"), device=0)
     good = g["status"] == 0
@@ -179,6 +177,12 @@ def test_gpu_whole_test_file_raw_signal_to_barcode_calls(g4000, models):
     want_fpt[g["stable_idx"]] = g["stable_fpt"]
     want_label[g["stable_idx"]] = g["stable_label"]
     assert set(g["stable_idx"].tolist()) <= set(g["tie_reads"].tolist()) and g["stable_idx"].size <= 2
+    # everything below is per read of the subset
+    want_fpt, want_label, good = want_fpt[idx], want_label[idx], good[idx]
+    g = dict(g)
+    for key in ("read_ids", "full_lengths", "calibration_offset", "calibration_scale", "cnn_preds", "success", "bounds", "path",
+                "status", "fail_reason"):
+        g[key] = g[key][idx]
     mismatches = {}
     # (the third pass: the sequential form of the step, without the fingerprint pass next to the LLR tail)
     for mode, inp, overlap in (("guarded", "float", True), ("exact", "adc", True), ("guarded", "adc", False)):
@@ -188,8 +192,8 @@ def test_gpu_whole_test_file_raw_signal_to_barcode_calls(g4000, models):
                                overlap_llr_tail=overlap)
         assert dmx.llr_fallback is None
         res = []
-        for lo in range(0, n, 1000):
-            sl = slice(lo, lo + 1000)
+        for lo in range(0, n, MINIBATCH):
+            sl = slice(lo, lo + MINIBATCH)
             batch = rows[sl] if inp == "float" else AdcBatch(adc[sl], num[sl], g["calibration_offset"][sl], g["calibration_scale"][sl])
             res.append(dmx.run(batch, g["full_lengths"][sl], g["read_ids"][sl], want_fpt=True))
         cat = lambda f: np.concatenate([getattr(r, f) for r in res])
@@ -206,14 +210,14 @@ def test_gpu_whole_test_file_raw_signal_to_barcode_calls(g4000, models):
             "label_failed_reads": np.flatnonzero(~good & (labels != -1)),
         }
         key = mode if overlap else mode + "_sequential"
-        mismatches[key] = {k: v.tolist() for k, v in bad.items() if v.size}
-        reasons = [res[i // 1000].fail_reason(i % 1000) or "" for i in np.flatnonzero(g["success"] == 0)]
+        mismatches[key] = {k: idx[v].tolist() for k, v in bad.items() if v.size}          # as read numbers of the file
+        reasons = [res[i // MINIBATCH].fail_reason(i % MINIBATCH) or "" for i in np.flatnonzero(g["success"] == 0)]
         want = [str(x) for x in g["fail_reason"][g["success"] == 0]]
         if reasons != want:
-            mismatches[key]["fail_reason"] = [(int(i), a, b) for i, a, b in zip(np.flatnonzero(g["success"] == 0), reasons, want) if a != b][:10]
+            mismatches[key]["fail_reason"] = [(int(i), a, b) for i, a, b in zip(idx[g["success"] == 0], reasons, want) if a != b][:10]
         df = res[0].predictions
-        assert list(df["#read_id"]) == [str(x) for x in g["read_ids"][:1000][good[:1000]]]
+        assert list(df["#read_id"]) == [str(x) for x in g["read_ids"][:MINIBATCH][good[:MINIBATCH]]]
         dmx.close()
     md.close()
     assert mismatches == {"guarded": {}, "exact": {}, "guarded_sequential": {}}, mismatches      # the mismatch list must be empty
-    assert (g["path"] == 2).sum() == 30 and (g["path"] == 1).sum() == 5 and g["success"].sum() == 3837
+    assert (g4000["path"] == 2).sum() == 30 and (g4000["path"] == 1).sum() == 5 and g4000["success"].sum() == 3837

@@ -36,7 +36,7 @@ def test_golden_inputs_are_reproducible(golden_fingerprint):
 def _ref_segmentation():
     hits = glob.glob(os.path.join(ROOT, "oracle", "_ref", "ref_c_segmentation*.so"))
     if not hits:
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref not built (oracle/build_ref.py needs a checkout of the reference, WDX_REFERENCE)")
     spec = importlib.util.spec_from_file_location("ref_c_segmentation", hits[0])
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)

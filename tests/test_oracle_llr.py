@@ -1,6 +1,6 @@
 """LLR fallback of the boundary detection (reference combined.py:222-296, llr.py, _c_llr.pyx).
 CPU: the restatement (oracle/wdx_oracle_llr.py) against (1) the reference's own compiled Cython gains
-(oracle/_ref/ref_c_llr, built by oracle/build_ref.py where /root/reference exists) and (2) the detection path,
+(oracle/_ref/ref_c_llr, built by oracle/build_ref.py from a checkout of the reference) and (2) the detection path,
 boundaries and verdicts the reference's `combined_detect_cnn` produced for the reads of
 test_data/demux/4000_rna004.pod5 that leave the plain CNN path (tests/golden/real4000_rna004_WDX4.npz,
 oracle/make_golden_real4000.py: 28 hail-mary validations, 193 LLR re-detections, 35 of them validating)."""
@@ -36,7 +36,7 @@ def llr_config(g):
 def test_gains_match_reference_cython():
     hits = glob.glob(os.path.join(ROOT, "oracle", "_ref", "ref_c_llr*.so"))
     if not hits:
-        pytest.skip("oracle/_ref/ref_c_llr not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/ref_c_llr not built (oracle/build_ref.py needs a checkout of the reference, WDX_REFERENCE)")
     spec = importlib.util.spec_from_file_location("ref_c_llr", hits[0])
     ref = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(ref)

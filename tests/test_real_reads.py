@@ -96,9 +96,14 @@ def test_pod5_reader_self_check():
 
 
 def test_pod5_reader_on_reference_file_if_present(golden_real):
-    path = "/root/reference/test_data/demux/4000_rna004.pod5"
+    """The pod5 reader on a file written by the pod5 library itself: the reference's test file, which is not part of this
+    repository (WDX_REFERENCE points at a checkout of the reference).  No cut-down copy is stored: none was taken from
+    that file, and a file written by this project's own code would check the reader only against itself; the decoder
+    keeps its synthetic self-check above."""
+    ref = os.environ.get("WDX_REFERENCE")
+    path = os.path.join(ref, "test_data", "demux", "4000_rna004.pod5") if ref else ""
     if not os.path.exists(path):
-        pytest.skip("reference test data not present (GPU box)")
+        pytest.skip("the reference's test_data/demux/4000_rna004.pod5 is not at hand (set WDX_REFERENCE)")
     from warpdemux_b200.io.pod5_min import Pod5File
 
     f = Pod5File(path)
