@@ -469,6 +469,41 @@ int wdx_validate_set_llr(wdx_validate* v, const wdx_llr_config* cfg);
 int wdx_calibrate_rows(const int16_t* adc, int64_t n, int64_t stride_in, const int32_t* n_valid, const float* offset,
                        const float* scale, float* out, int64_t stride_out, int device, void* stream);
 
+/* ---- pod5 VBZ signal -> int16 ADC rows on the device ----------------------------------------------------------
+ * A pod5 signal chunk is zstd( streamvbyte16( zigzag( delta( int16 )))), one zstd frame per chunk (RFC 8878).  The
+ * chunks go to the device still compressed; one warp decodes one frame, one CTA turns one read's chunks into its row.
+ * Supported zstd subset: one frame per chunk (single-segment or with a window descriptor, with or without
+ * Frame_Content_Size), raw / RLE / compressed blocks, raw / RLE / Huffman (1 or 4 streams) / treeless literals,
+ * predefined / RLE / FSE / repeat sequence tables.  Anything else is a per-chunk status, never a fault: */
+enum {
+    WDX_VBZ_OK = 0,
+    WDX_VBZ_BAD_MAGIC = 1,   /* not a zstd frame */
+    WDX_VBZ_DICTIONARY = 2,  /* the frame names a dictionary */
+    WDX_VBZ_CHECKSUM = 3,    /* content checksum flag set (not verified, so not accepted) */
+    WDX_VBZ_RESERVED = 4,    /* reserved header bit, block type or field */
+    WDX_VBZ_TRUNCATED = 5,   /* the input ends inside the frame */
+    WDX_VBZ_CORRUPT = 6,     /* inconsistent table description, bitstream, offset or size */
+    WDX_VBZ_TOO_LARGE = 7,   /* content larger than the output capacity (rows: the svb16 bound ceil(s/8) + 2 s) */
+    WDX_VBZ_FRAMES = 8,      /* skippable frame, or bytes after the frame (a second frame) */
+    WDX_VBZ_SAMPLES = 9,     /* rows: the key / data lengths disagree with the chunk's `samples` */
+    WDX_VBZ_SCRATCH = 10     /* rows: a chunk's scratch region is misaligned or smaller than it needs */
+};
+/* Decompress m frames: frame i = src[chunk_off[i], chunk_off[i+1]) -> scratch[scratch_off[i], scratch_off[i+1]).
+ * Decoding stops once limit[i] bytes exist (a prefix); content that exceeds the region while limit[i] is larger is
+ * WDX_VBZ_TOO_LARGE.  produced [m] int64 = bytes written (0 unless status is WDX_VBZ_OK), status [m] int32.
+ * DEVICE pointers; asynchronous on `stream`. */
+int wdx_zstd_decompress(const uint8_t* src, const int64_t* chunk_off, int64_t m, const int64_t* limit, uint8_t* scratch,
+                        const int64_t* scratch_off, int64_t* produced, int32_t* status, int device, void* stream);
+/* n reads of VBZ chunks -> int16 rows [n, stride]: read r = chunks [read_chunks[r], read_chunks[r+1]) in order, chunk c
+ * holds samples[c] samples; each chunk's delta sum restarts at 0 (pod5 decodes chunks independently).  Only the prefix
+ * of a chunk the row needs is decompressed.  Chunk c's scratch region [scratch_off[c], scratch_off[c+1]) must start
+ * 16-byte aligned and hold 16 + ceil(s/8) + 2 min(s, stride - first sample of c) bytes.  n_valid [n] int32 =
+ * min(sum of the read's samples, stride); samples beyond it are 0.  status [n] int32 = the first WDX_VBZ_* of the
+ * read's chunks; a read with a non-zero status has n_valid 0 and a zero row.  DEVICE pointers; asynchronous. */
+int wdx_vbz_decode_rows(const uint8_t* src, const int64_t* chunk_off, const int32_t* samples, int64_t m, const int64_t* read_chunks,
+                        int64_t n, uint8_t* scratch, const int64_t* scratch_off, int16_t* rows, int64_t stride, int32_t* n_valid,
+                        int32_t* status, int device, void* stream);
+
 /* ---- introspection -------------------------------------------------------- */
 const char* wdx_last_error(void);
 int wdx_device_count(void);

@@ -26,6 +26,7 @@ EXPORTS = [
     "wdx_cnn_create", "wdx_cnn_destroy", "wdx_cnn_detect", "wdx_cnn_prepare", "wdx_cnn_predict", "wdx_cnn_score_len", "wdx_cnn_set_guard", "wdx_cnn_enable_timing",
     "wdx_cnn_last_kernel_ms",
     "wdx_validate_create", "wdx_validate_destroy", "wdx_validate_run", "wdx_validate_enable_timing", "wdx_validate_last_kernel_ms", "wdx_validate_set_verdict_only", "wdx_validate_set_early", "wdx_validate_run_ex", "wdx_validate_run_report", "wdx_calibrate_rows", "wdx_validate_set_llr",
+    "wdx_zstd_decompress", "wdx_vbz_decode_rows",
 ]
 
 _lib = None
@@ -151,6 +152,10 @@ def load():
         L.wdx_validate_run_report.argtypes = [vp, vp, i64, i64, vp, vp, i32, vp, vp, vp, vp, vp, vp, vp]
         L.wdx_calibrate_rows.restype = i32
         L.wdx_calibrate_rows.argtypes = [vp, i64, i64, vp, vp, vp, vp, i64, i32, vp]
+        L.wdx_zstd_decompress.restype = i32
+        L.wdx_zstd_decompress.argtypes = [vp, vp, i64, vp, vp, vp, vp, vp, i32, vp]
+        L.wdx_vbz_decode_rows.restype = i32
+        L.wdx_vbz_decode_rows.argtypes = [vp, vp, vp, i64, vp, i64, vp, vp, vp, i64, vp, vp, i32, vp]
         L.wdx_validate_set_verdict_only.restype = i32
         L.wdx_validate_set_verdict_only.argtypes = [vp, i32]
         L.wdx_validate_set_early.restype = i32

@@ -15,8 +15,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libwdx_b200.so")
-SOURCES = ["wdx_b200.cu", "wdx_fp.cu", "wdx_cnn.cu", "wdx_validate.cu"]
-HEADERS = ["wdx_types.cuh", "fused_kernels.cuh", "dtw_band.cuh", "dtw_band_x2.cuh", "dtw_wavefront.cuh", "fingerprint_kernel.cuh", "wdx_internal.cuh", "cnn_kernels.cuh", "block_select.cuh", "cnn_tc_kernel.cuh", "validate_kernel.cuh", "llr_kernel.cuh",
+SOURCES = ["wdx_b200.cu", "wdx_fp.cu", "wdx_cnn.cu", "wdx_validate.cu", "wdx_vbz.cu"]
+HEADERS = ["wdx_types.cuh", "fused_kernels.cuh", "dtw_band.cuh", "dtw_band_x2.cuh", "dtw_wavefront.cuh", "fingerprint_kernel.cuh", "wdx_internal.cuh", "cnn_kernels.cuh", "block_select.cuh", "cnn_tc_kernel.cuh", "validate_kernel.cuh", "llr_kernel.cuh", "vbz_kernel.cuh",
            os.path.join("..", "..", "include", "wdx_b200.h")]
 
 NVCC_FLAGS = [

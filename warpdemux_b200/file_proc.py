@@ -26,6 +26,7 @@ import numpy as np
 import pandas as pd
 
 from . import _lib
+from . import vbz as _vbz
 from .detect import cnn as _cnn
 from .detect import combined as _combined
 from .models.utils import predictions_to_df
@@ -51,6 +52,20 @@ class AdcBatch:
     num_samples: np.ndarray    # [n] samples present per row (min(read length, stride))
     offset: np.ndarray         # float32 [n] calibration_offset
     scale: np.ndarray          # float32 [n] calibration_scale
+
+
+@dataclass
+class VbzBatch:
+    """A minibatch as the still-compressed pod5 signal chunks of its reads (`io.pod5_min.Pod5File.vbz_minibatches`):
+    the chunks go to the device as they are and are decoded there into the int16 rows an `AdcBatch` carries
+    (`vbz.decode_rows`), then calibrated like them.  Read r = chunks read_chunks[r] .. read_chunks[r+1]-1 in order."""
+    data: np.ndarray           # uint8 [bytes] the chunks' zstd frames, concatenated
+    chunk_offsets: np.ndarray  # int64 [m+1] frame c = data[chunk_offsets[c]:chunk_offsets[c+1]]
+    chunk_samples: np.ndarray  # int32 [m] samples of chunk c (the pod5 signal table's `samples`)
+    read_chunks: np.ndarray    # int64 [n+1] CSR: the chunks of each read
+    offset: np.ndarray         # float32 [n] calibration_offset
+    scale: np.ndarray          # float32 [n] calibration_scale
+    stride: int                # row length (the preload size); chunks past it are not needed
 
 
 @dataclass
@@ -183,6 +198,8 @@ class MinibatchDemuxer:
         job = {"slot": slot, "read_ids": read_ids}
         if isinstance(signals, AdcBatch):
             return self._upload_adc(job, signals, full_lengths)
+        if isinstance(signals, VbzBatch):
+            return self._upload_vbz(job, signals, full_lengths)
         if isinstance(signals, torch.Tensor):
             if signals.dtype != torch.float32 or signals.dim() != 2 or not signals.is_contiguous():
                 raise ValueError("signals tensor must be contiguous float32 [n, stride]")
@@ -256,6 +273,64 @@ class MinibatchDemuxer:
         job.update(d_sig=d_sig, d_len=d_len, ev_h2d=ev, h2d_bytes=int(n) * int(stride) * 2)
         return job
 
+    def _upload_vbz(self, job: dict, b: VbzBatch, full_lengths) -> dict:
+        """Phase 1 for pod5 VBZ chunks: the compressed bytes and the small arrays go up from one pinned staging block
+        (two copies), then wdx_vbz_decode_rows -> int16 rows -> wdx_calibrate_rows, all on the copy stream.  The per-read
+        decode status joins the result block (_launch) and is checked in _finalize."""
+        torch = self._torch
+        st, cst = self._streams()
+        slot = job["slot"]
+        stride = int(b.stride)
+        rc = np.ascontiguousarray(b.read_chunks, dtype=np.int64).reshape(-1)
+        n = rc.size - 1
+        samples = np.ascontiguousarray(b.chunk_samples, dtype=np.int32).reshape(-1)
+        coff = np.ascontiguousarray(b.chunk_offsets, dtype=np.int64).reshape(-1)
+        data = np.asarray(b.data, dtype=np.uint8).reshape(-1)
+        if stride < 1 or n < 0 or coff.size != samples.size + 1 or (coff.size and (coff[0] != 0 or coff[-1] != data.size or np.any(np.diff(coff) < 0))):
+            raise ValueError("VbzBatch: chunk_offsets must be [m+1] non-decreasing offsets into data, chunk_samples [m], stride >= 1")
+        soff = _vbz.scratch_layout(samples, rc, stride)
+        lens = np.ascontiguousarray(np.minimum(np.asarray(full_lengths, dtype=np.int64).reshape(-1), np.iinfo(np.int32).max), dtype=np.int32)
+        if lens.shape[0] != n:
+            raise ValueError("full_lengths must have one entry per read")
+        # small arrays: one int64-aligned block
+        parts = [("coff", coff), ("soff", soff), ("rc", rc), ("samples", samples), ("len", lens),
+                 ("offset", np.asarray(b.offset, dtype=np.float32).reshape(-1)), ("scale", np.asarray(b.scale, dtype=np.float32).reshape(-1))]
+        if parts[5][1].size != n or parts[6][1].size != n:
+            raise ValueError("VbzBatch: offset / scale need one entry per read")
+        at, pos = {}, 0
+        for name, a in parts:
+            at[name] = (pos, a)
+            pos += (a.nbytes + 15) // 16 * 16
+        nbytes_data = (data.size + 15) // 16 * 16
+        job.update(n=n, stride=stride, lens=lens, h_sig=None)
+        with torch.cuda.stream(cst):
+            pin = self._pinned(f"{slot}:vbz", nbytes_data + pos, torch.uint8)
+            hp = pin.numpy()
+            hp[:data.size] = data
+            for name, (o, a) in at.items():
+                hp[nbytes_data + o:nbytes_data + o + a.nbytes] = a.view(np.uint8)
+            d_bytes = self._get(f"{slot}:vbz_bytes", (max(nbytes_data, 16),), torch.uint8)
+            d_small = self._get(f"{slot}:vbz_small", (max(pos, 16),), torch.uint8)
+            if nbytes_data:
+                d_bytes[:nbytes_data].copy_(pin[:nbytes_data], non_blocking=True)
+            d_small[:pos].copy_(pin[nbytes_data:nbytes_data + pos], non_blocking=True)
+            tdt = {np.dtype(np.int64): torch.int64, np.dtype(np.int32): torch.int32, np.dtype(np.float32): torch.float32}
+            v = {name: d_small[o:o + a.nbytes].view(tdt[a.dtype]) for name, (o, a) in at.items()}
+            d_scr = self._get(f"{slot}:vbz_scratch", (max(int(soff[-1]), 16),), torch.uint8)
+            d_adc = self._get(f"{slot}:adc", (n, stride), torch.int16)
+            d_dec = self._get(f"{slot}:vbz_dec", (2, n), torch.int32)    # n_valid, status
+            d_sig = self._get(f"{slot}:sig", (n, stride), torch.float32)
+            if n:
+                _vbz.decode_rows_raw(d_bytes, v["coff"], v["samples"], v["rc"], d_scr, v["soff"], d_adc, d_dec[0], d_dec[1],
+                                     self.device, cst.cuda_stream)
+                rc_ = _lib.load().wdx_calibrate_rows(d_adc.data_ptr(), n, stride, d_dec[0].data_ptr(), v["offset"].data_ptr(),
+                                                     v["scale"].data_ptr(), d_sig.data_ptr(), stride, self.device, cst.cuda_stream)
+                _lib.check(rc_, "wdx_calibrate_rows")
+            ev = torch.cuda.Event()
+            ev.record(cst)
+        job.update(d_sig=d_sig, d_len=v["len"], ev_h2d=ev, d_vbz_status=d_dec[1], h2d_bytes=int(data.size) + pos)
+        return job
+
     def _launch(self, job: dict, want_fpt: bool) -> None:
         """Phase 2 (the lane's compute stream): CNN -> validation / LLR -> fingerprint + DTW/SVC, then the result download."""
         torch = self._torch
@@ -275,6 +350,8 @@ class MinibatchDemuxer:
                     ("status", (n,), torch.int32), ("suc", (n,), torch.uint8), ("flags", (n,), torch.uint8)]
             if want_fpt:
                 spec.insert(0, ("fpt", (n, L), torch.float64))
+            if "d_vbz_status" in job:
+                spec.append(("vbz_status", (n,), torch.int32))
             sizes = [(int(np.prod(shape)) * torch.empty(0, dtype=dt).element_size() + 7) // 8 * 8 for _, shape, dt in spec]
             total = sum(sizes)
             d_block = g("results", (max(total, 8),), torch.uint8)
@@ -291,6 +368,8 @@ class MinibatchDemuxer:
             if d_fpt is None:     # kept on the device anyway: a guard-list overflow is repaired from it (_finalize)
                 d_fpt = g("fpt_dev", (n, L), torch.float64)
             d_flags = views["flags"]
+            if "d_vbz_status" in job:
+                views["vbz_status"].copy_(job["d_vbz_status"])
             d_a0, d_a1 = g("a0", (n,), torch.int64), g("a1", (n,), torch.int64)
             sp = st.cuda_stream
             rescued = np.zeros(n, dtype=bool)
@@ -350,6 +429,13 @@ class MinibatchDemuxer:
         """Phase 3 (host): wait for the download, copy out of the pinned blocks, build the DataFrame."""
         job["ev_done"].synchronize()
         h = {k: v.numpy().copy() for k, v in job["host"].items()}
+        if "vbz_status" in h and h["vbz_status"].any():
+            # a pod5 chunk that does not decode is an I/O error of the input file, not a per-read verdict
+            bad = np.flatnonzero(h["vbz_status"])
+            rid = job["read_ids"]
+            name = lambda i: rid[i] if rid is not None else f"row {i}"
+            raise _lib.WdxError(f"read {name(bad[0])}: VBZ signal could not be decoded ({_vbz.status_name(h['vbz_status'][bad[0]])}, "
+                                f"status {int(h['vbz_status'][bad[0]])}); {bad.size} of {job['n']} reads of the minibatch failed")
         labels, conf, prob, status = h["lab"], h["conf"], h["prob"], h["status"]
         flags = h["flags"]
         over = np.flatnonzero((flags & _lib.FLAG_GUARD_OVERFLOW) != 0)
@@ -391,7 +477,8 @@ class MinibatchDemuxer:
     def run(self, signals, full_lengths, read_ids: Optional[Sequence] = None, return_df: bool = True,
             want_fpt: bool = False) -> MinibatchResult:
         """One minibatch.  signals: float32 [n, stride] NaN-padded rows (numpy; torch CPU tensor, pinned or not; or a CUDA
-        tensor), or an `AdcBatch` of raw int16 samples; full_lengths: [n] full read lengths (file_proc.py:241-262)."""
+        tensor), an `AdcBatch` of raw int16 samples or a `VbzBatch` of compressed pod5 signal chunks (a chunk that does
+        not decode raises WdxError naming the read); full_lengths: [n] full read lengths (file_proc.py:241-262)."""
         with self._torch.cuda.device(self.device):
             job = self._upload(0, signals, full_lengths, read_ids)
             self._launch(job, want_fpt)

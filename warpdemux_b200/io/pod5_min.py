@@ -50,6 +50,26 @@ def decode_vbz(chunk: bytes, n_samples: int) -> np.ndarray:
     return np.cumsum(zz, dtype=np.int32).astype(np.int16)            # delta (wraps like int16 arithmetic)
 
 
+def _uuid_strings(col) -> np.ndarray:
+    """A column of 16-byte read ids -> str [n] in uuid.UUID's canonical form, without a per-read Python loop."""
+    import pyarrow as pa
+
+    arr = col.combine_chunks() if isinstance(col, pa.ChunkedArray) else col
+    if isinstance(arr, pa.ExtensionArray):
+        arr = arr.storage
+    if pa.types.is_fixed_size_binary(arr.type):
+        raw = np.frombuffer(arr.buffers()[1], dtype=np.uint8)[arr.offset * 16:(arr.offset + len(arr)) * 16]
+    else:
+        raw = np.frombuffer(b"".join(arr.to_pylist()), dtype=np.uint8)
+    raw = raw.reshape(-1, 16)
+    hexd = np.frombuffer(b"0123456789abcdef", dtype=np.uint8)[np.stack([raw >> 4, raw & 15], axis=-1).reshape(-1, 32)]
+    out = np.full((raw.shape[0], 36), ord("-"), dtype=np.uint8)
+    for dst, src in ((slice(0, 8), slice(0, 8)), (slice(9, 13), slice(8, 12)), (slice(14, 18), slice(12, 16)),
+                     (slice(19, 23), slice(16, 20)), (slice(24, 36), slice(20, 32))):
+        out[:, dst] = hexd[:, src]
+    return out.view("S36").ravel().astype(str)
+
+
 @dataclass
 class Pod5Read:
     read_id: str
@@ -116,6 +136,72 @@ class Pod5File:
     def _signal(self, rows: Sequence[int]) -> np.ndarray:
         parts = [self._signal_row(int(r)) for r in rows]
         return parts[0] if len(parts) == 1 else np.concatenate(parts)
+
+    def _vbz_index(self):
+        """The signal table as one large_binary column (storage of the `minknow.vbz` extension type) with its offsets and
+        bytes as numpy views, and its `samples`; the reads table's flattened signal-row lists.  Built once."""
+        if getattr(self, "_vbz", None) is None:
+            import pyarrow as pa
+
+            cols, samples = [], []
+            for i in range(self._sig.num_record_batches):
+                b = self._sig.get_batch(i)
+                col = b.column("signal")
+                if isinstance(col, pa.ExtensionArray):
+                    col = col.storage
+                cols.append(col if col.type == pa.large_binary() else col.cast(pa.large_binary()))
+                samples.append(np.asarray(b.column("samples").to_numpy(zero_copy_only=False), dtype=np.int64))
+            rows = self._reads.column("signal").combine_chunks()
+            if isinstance(rows, pa.ExtensionArray):
+                rows = rows.storage
+            loff = rows.offsets.to_numpy().astype(np.int64)
+            sig = pa.concat_arrays(cols) if cols else pa.array([], type=pa.large_binary())
+            off = np.frombuffer(sig.buffers()[1], dtype=np.int64)[sig.offset:sig.offset + len(sig) + 1]
+            data = np.frombuffer(sig.buffers()[2], dtype=np.uint8) if len(sig) else np.zeros(0, np.uint8)
+            self._vbz = dict(signal=sig, off=off, data=data,
+                             samples=np.concatenate(samples) if samples else np.zeros(0, np.int64),
+                             row_off=loff - loff[0], rows=np.asarray(rows.flatten().to_numpy(zero_copy_only=False), dtype=np.int64))
+        return self._vbz
+
+    def vbz_minibatches(self, batch_size: int = 1000, preload: int = 11500):
+        """Minibatches of still-compressed signal for the device decoder: yields (file_proc.VbzBatch, full_lengths
+        int64 [n] (= num_samples), read_ids [n] str) per `batch_size` reads in file order.  A read keeps the chunks that
+        start below `preload` samples (the row length); their bytes are not decoded here: a minibatch whose chunks are
+        consecutive signal-table rows gets a view of the column's bytes, other minibatches a gather by Arrow (`take`)."""
+        import pyarrow as pa
+
+        from ..file_proc import VbzBatch
+
+        ix = self._vbz_index()
+        t = self._reads
+        num = np.asarray(t.column("num_samples").to_numpy(), dtype=np.int64)
+        cal_off = np.asarray(t.column("calibration_offset").to_numpy(), dtype=np.float32)
+        cal_sc = np.asarray(t.column("calibration_scale").to_numpy(), dtype=np.float32)
+        ids = _uuid_strings(t.column("read_id"))
+        loff, rows_all, samples_all = ix["row_off"], ix["rows"], ix["samples"]
+        for a in range(0, t.num_rows, int(batch_size)):
+            b = min(a + int(batch_size), t.num_rows)
+            nr = b - a
+            rows = rows_all[loff[a]:loff[b]]
+            cnt = np.diff(loff[a:b + 1])
+            s = samples_all[rows]
+            read_of = np.repeat(np.arange(nr), cnt)
+            excl = np.cumsum(s) - s
+            first = (loff[a:b] - loff[a])[read_of]
+            keep = (excl - excl[first]) < preload if rows.size else np.zeros(0, dtype=bool)
+            rc = np.concatenate([[0], np.cumsum(np.bincount(read_of[keep], minlength=nr))]).astype(np.int64)
+            r = rows[keep]
+            if r.size == 0 or np.all(np.diff(r) == 1):     # the usual layout: the minibatch's chunks are consecutive rows
+                lo_, hi_ = (r[0], r[-1] + 1) if r.size else (0, 0)
+                off = ix["off"][lo_:hi_ + 1]
+                data = ix["data"][off[0]:off[-1]] if r.size else np.zeros(0, np.uint8)
+            else:
+                sel = ix["signal"].take(pa.array(r, type=pa.int64()))
+                off = np.frombuffer(sel.buffers()[1], dtype=np.int64)[sel.offset:sel.offset + len(sel) + 1]
+                data = np.frombuffer(sel.buffers()[2], dtype=np.uint8)[off[0]:off[-1]]
+            batch = VbzBatch(data=data, chunk_offsets=(off - off[0]).astype(np.int64), chunk_samples=s[keep].astype(np.int32),
+                             read_chunks=rc, offset=cal_off[a:b], scale=cal_sc[a:b], stride=int(preload))
+            yield batch, num[a:b].copy(), ids[a:b]
 
     def reads(self, selection: Optional[Sequence[str]] = None) -> Iterator[Pod5Read]:
         t = self._reads
