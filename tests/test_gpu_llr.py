@@ -148,6 +148,48 @@ def _spc(g):
                            cnn_boundaries=cnn.CNNBoundariesConfig(polya_cand_k=c["polya_cand_k"]))
 
 
+def whole_file_expectations(g, idx):
+    """The reference chain's whole-file results for the reads `idx` of real4000_rna004_WDX4.npz (read numbers of the file,
+    repeats allowed): CNN predictions, detection verdict, boundaries, path, fingerprint status, fail reasons, fingerprints
+    and barcode calls.  Where numpy's unstable argsort of EQUAL t-test scores decided the change points on the machine that
+    wrote the fixture, the expected fingerprint and call are the oracle's stable-order ones (`stable_idx`)."""
+    good = g["status"] == 0
+    pos = np.cumsum(good) - 1
+    want_fpt, want_label = g["fpt"].copy(), np.where(good, g["y_pred"][np.maximum(pos, 0)], -1)
+    want_fpt[g["stable_idx"]] = g["stable_fpt"]
+    want_label[g["stable_idx"]] = g["stable_label"]
+    assert set(g["stable_idx"].tolist()) <= set(g["tie_reads"].tolist()) and g["stable_idx"].size <= 2
+    want = {key: g[key][idx] for key in ("read_ids", "full_lengths", "calibration_offset", "calibration_scale", "cnn_preds", "success",
+                                         "bounds", "path", "status", "fail_reason")}
+    want.update(fpt=want_fpt[idx], label=want_label[idx], good=good[idx])
+    return want
+
+
+def chain_mismatches(want, res):
+    """MinibatchResults `res` (in order, want_fpt=True) against `whole_file_expectations` -> {field: row positions that differ}."""
+    cat = lambda f: np.concatenate([getattr(r, f) for r in res])
+    suc, bounds, preds = cat("detect_success"), cat("bounds"), cat("preds")
+    labels, status, fpt, src = cat("labels"), cat("fp_status"), cat("fpt"), cat("detect_source")
+    good = want["good"]
+    bad = {
+        "cnn_preds": np.flatnonzero((preds != want["cnn_preds"]).any(axis=1)),
+        "detect_success": np.flatnonzero(suc != want["success"]),
+        "bounds": np.flatnonzero((bounds != want["bounds"]).any(axis=1) & (want["success"] == 1)),
+        "path": np.flatnonzero(((src & 3) != want["path"]) & (want["success"] == 1)),
+        "fp_status": np.flatnonzero(status != want["status"]),
+        "fpt": np.flatnonzero(good & ~np.all(fpt == want["fpt"], axis=1)),
+        "label": np.flatnonzero(good & (labels != want["label"])),
+        "label_failed_reads": np.flatnonzero(~good & (labels != -1)),
+    }
+    out = {k: v for k, v in bad.items() if v.size}
+    reasons = [r.fail_reason(i) or "" for r in res for i in range(r.labels.size)]
+    failed = np.flatnonzero(want["success"] == 0)
+    wrong = [int(i) for i in failed if reasons[i] != str(want["fail_reason"][i])]
+    if wrong:
+        out["fail_reason"] = np.array(wrong)
+    return out
+
+
 def test_gpu_whole_test_file_raw_signal_to_barcode_calls(g4000, models):
     """BASELINE.json configs[0] on the reads of test_data/demux/4000_rna004.pod5 whose int16 rows the fixture keeps
     (every read that leaves the plain CNN path, every 16th read and the tie read below: 439 of the 4000), in minibatches
@@ -169,20 +211,9 @@ def test_gpu_whole_test_file_raw_signal_to_barcode_calls(g4000, models):
     assert set(np.flatnonzero(off_path).tolist()) | set(g["stable_idx"].tolist()) <= set(idx.tolist())
     spc = _spc(g)
     md = cnn.load_cnn_model(os.path.join(GOLD, "models", "cnn_rna004_130bps_v0.2.4.npz"), device=0)
-    good = g["status"] == 0
-    pos = np.cumsum(good) - 1
-    # the reference's expected fingerprints / calls; for the reads where numpy's unstable argsort of EQUAL t-test scores
-    # decided the change points on the machine that wrote the fixture, the stable-sort result (oracle, stable_ties)
-    want_fpt, want_label = g["fpt"].copy(), np.where(good, g["y_pred"][np.maximum(pos, 0)], -1)
-    want_fpt[g["stable_idx"]] = g["stable_fpt"]
-    want_label[g["stable_idx"]] = g["stable_label"]
-    assert set(g["stable_idx"].tolist()) <= set(g["tie_reads"].tolist()) and g["stable_idx"].size <= 2
     # everything below is per read of the subset
-    want_fpt, want_label, good = want_fpt[idx], want_label[idx], good[idx]
-    g = dict(g)
-    for key in ("read_ids", "full_lengths", "calibration_offset", "calibration_scale", "cnn_preds", "success", "bounds", "path",
-                "status", "fail_reason"):
-        g[key] = g[key][idx]
+    want = whole_file_expectations(g, idx)
+    good = want["good"]
     mismatches = {}
     # (the third pass: the sequential form of the step, without the fingerprint pass next to the LLR tail)
     for mode, inp, overlap in (("guarded", "float", True), ("exact", "adc", True), ("guarded", "adc", False)):
@@ -194,29 +225,12 @@ def test_gpu_whole_test_file_raw_signal_to_barcode_calls(g4000, models):
         res = []
         for lo in range(0, n, MINIBATCH):
             sl = slice(lo, lo + MINIBATCH)
-            batch = rows[sl] if inp == "float" else AdcBatch(adc[sl], num[sl], g["calibration_offset"][sl], g["calibration_scale"][sl])
-            res.append(dmx.run(batch, g["full_lengths"][sl], g["read_ids"][sl], want_fpt=True))
-        cat = lambda f: np.concatenate([getattr(r, f) for r in res])
-        suc, bounds, preds = cat("detect_success"), cat("bounds"), cat("preds")
-        labels, status, fpt, src = cat("labels"), cat("fp_status"), cat("fpt"), cat("detect_source")
-        bad = {
-            "cnn_preds": np.flatnonzero((preds != g["cnn_preds"]).any(axis=1)),
-            "detect_success": np.flatnonzero(suc != g["success"]),
-            "bounds": np.flatnonzero((bounds != g["bounds"]).any(axis=1) & (g["success"] == 1)),
-            "path": np.flatnonzero(((src & 3) != g["path"]) & (g["success"] == 1)),
-            "fp_status": np.flatnonzero(status != g["status"]),
-            "fpt": np.flatnonzero(good & ~np.all(fpt == want_fpt, axis=1)),
-            "label": np.flatnonzero(good & (labels != want_label)),
-            "label_failed_reads": np.flatnonzero(~good & (labels != -1)),
-        }
+            batch = rows[sl] if inp == "float" else AdcBatch(adc[sl], num[sl], want["calibration_offset"][sl], want["calibration_scale"][sl])
+            res.append(dmx.run(batch, want["full_lengths"][sl], want["read_ids"][sl], want_fpt=True))
         key = mode if overlap else mode + "_sequential"
-        mismatches[key] = {k: idx[v].tolist() for k, v in bad.items() if v.size}          # as read numbers of the file
-        reasons = [res[i // MINIBATCH].fail_reason(i % MINIBATCH) or "" for i in np.flatnonzero(g["success"] == 0)]
-        want = [str(x) for x in g["fail_reason"][g["success"] == 0]]
-        if reasons != want:
-            mismatches[key]["fail_reason"] = [(int(i), a, b) for i, a, b in zip(idx[g["success"] == 0], reasons, want) if a != b][:10]
+        mismatches[key] = {k: idx[v].tolist() for k, v in chain_mismatches(want, res).items()}      # as read numbers of the file
         df = res[0].predictions
-        assert list(df["#read_id"]) == [str(x) for x in g["read_ids"][:MINIBATCH][good[:MINIBATCH]]]
+        assert list(df["#read_id"]) == [str(x) for x in want["read_ids"][:MINIBATCH][good[:MINIBATCH]]]
         dmx.close()
     md.close()
     assert mismatches == {"guarded": {}, "exact": {}, "guarded_sequential": {}}, mismatches      # the mismatch list must be empty

@@ -41,6 +41,7 @@ class DeviceModel:
             int(p.pwr_dist), self.device, C.byref(h))
         _lib.check(rc, "wdx_model_create")
         self._h = h
+        self.thresholds = p.thresholds   # the array uploaded; a holder of `params` rebuilds when it is replaced
 
     def close(self):
         if getattr(self, "_h", None):

@@ -97,6 +97,10 @@ class BaseDTWModel(ABC):
             self._dev = None
 
     def _device_model(self):
+        # the thresholds are applied on the device: when another holder of the same params replaced them (the lanes of
+        # MinibatchDemuxer share lane 0's params), this replica rebuilds too
+        if self._dev is not None and self._dev.thresholds is not self.params.thresholds:
+            self._drop_device()
         if self._dev is None:
             from ..device_model import DeviceModel
             from ..sharding import default_device
